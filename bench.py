@@ -17,6 +17,11 @@ available offline): 5.8 M seeded Gaussians tuned to M/N ~ 5 (SURVEY 8d).
   --impl reference : the reference has no CPU path and its Vulkan build is unavailable here, so
           the reference arm times the CPU oracle (oracle/, "port") on the box's host cores on a
           bounded sample (a band of tile rows of the same frame) and extrapolates frames/s.
+  --dump-outputs DIR : after the timed frames, writes the framebuffer the last timed frame produced
+          to DIR/frame_bgra8.npy as float32 (H, W, 4), so that two builds run with the same arguments
+          can be compared output for output.  A frame larger than DUMP_BUDGET_BYTES is written as a
+          fixed, seeded sample of whole pixels: frame_bgra8.npy (K, 4) and their row-major pixel
+          indices in frame_pixel_index.npy (K,) float64.
 """
 from __future__ import annotations
 
@@ -50,6 +55,8 @@ WORKLOADS = {
                note="BASELINE config 1: synthetic 10k, 640x480"),
 }
 NUM_CAMERAS = 8  # small orbit so consecutive frames differ (M varies a few %)
+DUMP_BUDGET_BYTES = 60_000_000  # --dump-outputs writes at most this much (plus .npy headers)
+DUMP_SEED = 0
 
 
 def make_scene(g, wl, first=0, count=None):
@@ -136,6 +143,20 @@ def measured_peak_gbs():
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
 
 
+def dump_frame(out_dir, frame):
+    """Writes an (H, W, 4) uint8 framebuffer as float32 .npy files in out_dir (see --dump-outputs in the docstring)."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    px = frame.reshape(-1, frame.shape[-1])
+    if px.size * 4 <= DUMP_BUDGET_BYTES:
+        np.save(out_dir / "frame_bgra8.npy", frame.astype(np.float32))
+        return
+    k = DUMP_BUDGET_BYTES // (px.shape[1] * 4 + 8)  # float32 channels + one float64 index per pixel
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(px.shape[0], size=k, replace=False))
+    np.save(out_dir / "frame_bgra8.npy", px[idx].astype(np.float32))
+    np.save(out_dir / "frame_pixel_index.npy", idx.astype(np.float64))
+
+
 def use_all_cores(o):
     """torchrun exports OMP_NUM_THREADS=1 to its workers; the CPU baseline should use every core this process may run on."""
     try:
@@ -198,7 +219,13 @@ def main():
     ap.add_argument("--sh16", action="store_true", help="gsb_set_sh_storage(1): fp16 SH coefficients -- NOT a parity mode, never the default")
     ap.add_argument("--no-extra", action="store_true", help="skip the C4 / C5 extra workload measured at --gpus 4 / 8")
     ap.add_argument("--tile-cull", type=int, default=2, help="gsb_set_tile_cull level: 0 reference lists, 1 exact per-tile instance culling, 2 coarse bins (image bit-identical in all three)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the framebuffer of the last timed frame to DIR/*.npy (float32; sampled above DUMP_BUDGET_BYTES)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times frames that keep no image")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -289,6 +316,8 @@ def main():
                 out["extra_workloads"] = [{"workload": extra_name, "error": repr(exc)}]
     if rank == 0:
         print(json.dumps(out))
+        if args.dump_outputs:
+            dump_frame(args.dump_outputs, env["last_frame"])
     ctx.close()
     if world > 1:
         dist.destroy_process_group()
@@ -403,6 +432,9 @@ def measure(env, wl_name, wl, steps, warmup, headline):
     barrier()
     ms_step = reduce_max(e0.elapsed_time(e1)) / steps
     ctx.stats()  # raises GSB_ERR_OVERFLOW if any async frame overflowed the arena (sticky flag)
+    if headline and args.dump_outputs and rank == 0:  # the last timed frame, before later loops overwrite it
+        src = torch.as_tensor(_DevFrame(ctx.frame_ptr(), (H, W, bpp)), device=dev) if sharded else dev_fb[0]
+        env["last_frame"] = src.cpu().numpy()
 
     # ---- per-frame distribution (SURVEY 8d: median / p95): the same frames again with an event after every frame ----
     nd = min(steps, 200)
