@@ -1,14 +1,15 @@
 // gs_viewer_headless -- the reference viewer's command line (apps/viewer/main.cpp:12-98) without a window:
 //   gs_viewer_headless [-d DEVICE] [-w WIDTH] [-h HEIGHT] [-v] [--frames N] [--camera x,y,z[,qw,qx,qy,qz]]
 //                      [--fov DEG] [--camera-path poses.txt] [--mode exact|fast] [--cull [LEVEL]] [--out image.ppm]
-//                      [--float-out image.pfm] scene.ply
+//                      [--float-out image.pfm] [--alpha-out alpha.pfm] [--depth-out depth.pfm] scene.ply
 // --camera-path: one pose per line `x y z qw qx qy qz [fov]` (# comments); `--frames` frames are rendered at each pose
 // and one JSON line is printed per pose (SURVEY 8d: record M for every timed camera).
 // Loads the .ply through GSScene, renders N frames through Renderer::draw() (B8G8R8A8 like the swapchain),
 // prints the six per-stage timers + `instances` (Renderer.cpp:85-100,540) as one JSON line per run and
 // optionally writes the last frame as a binary PPM (8-bit, what the swapchain would show) and / or as a PFM (float32 RGB, the
 // unquantised blend render.comp:98 stores: what the 1e-4 parity tolerance is defined on).  The first JSON line also carries
-// the load times (file read + activation, upload + cov3D ingest).  Environment: VKGS_PHYSICAL_DEVICE like the viewer.
+// the load times (file read + activation, upload + cov3D ingest).  --alpha-out / --depth-out write the opacity (1 - final
+// transmittance) and the un-normalised expected depth of one Renderer::renderAux frame as greyscale PFMs ("Pf", bottom to top).  Environment: VKGS_PHYSICAL_DEVICE like the viewer.
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -23,12 +24,12 @@
 static void usage() {
     std::puts("usage: gs_viewer_headless [-d device] [-w width] [-h height] [-v] [--frames n] [--camera x,y,z[,qw,qx,qy,qz]]\n"
               "                          [--fov deg] [--camera-path poses.txt] [--mode exact|fast] [--cull [0|1|2]] [--out image.ppm]\n"
-              "                          [--float-out image.pfm] scene.ply");
+              "                          [--float-out image.pfm] [--alpha-out alpha.pfm] [--depth-out depth.pfm] scene.ply");
 }
 
 int main(int argc, char** argv) {
     Renderer::Configuration cfg;
-    std::string out_path, float_path, scene, path_file;
+    std::string out_path, float_path, alpha_path, depth_path, scene, path_file;
     int cull_level = 0;
     uint32_t frames = 1;
     bool verbose = false, cull = false;
@@ -56,6 +57,8 @@ int main(int argc, char** argv) {
             cull_level = 1;
             if (i + 1 < argc && std::strlen(argv[i + 1]) == 1 && argv[i + 1][0] >= '0' && argv[i + 1][0] <= '2') cull_level = argv[++i][0] - '0';
         } else if (a == "--float-out") float_path = next();
+        else if (a == "--alpha-out") alpha_path = next();
+        else if (a == "--depth-out") depth_path = next();
         else if (a == "--out") out_path = next();
         else if (a == "--camera-path") path_file = next();
         else if (a == "--camera") {
@@ -137,6 +140,20 @@ int main(int argc, char** argv) {
                 for (uint32_t x = 0; x < cfg.width; x++)
                     for (int c = 0; c < 3; c++) row[x * 3 + c] = px[(static_cast<size_t>(y) * cfg.width + x) * 4 + c];
                 f.write(reinterpret_cast<const char*>(row.data()), static_cast<std::streamsize>(row.size() * sizeof(float)));
+            }
+        }
+        if (!alpha_path.empty() || !depth_path.empty()) {  // one renderAux frame: (opacity, expected depth) per pixel
+            const float* aux = renderer.renderAux(cfg.width, cfg.height, cfg.format);
+            for (int plane = 0; plane < 2; plane++) {
+                const std::string& path = plane == 0 ? alpha_path : depth_path;
+                if (path.empty()) continue;
+                std::ofstream f(path, std::ios::binary);  // greyscale PFM: "Pf", rows bottom to top like --float-out
+                f << "Pf\n" << cfg.width << " " << cfg.height << "\n-1.0\n";
+                std::vector<float> row(cfg.width);
+                for (uint32_t y = cfg.height; y-- > 0;) {
+                    for (uint32_t x = 0; x < cfg.width; x++) row[x] = aux[(static_cast<size_t>(y) * cfg.width + x) * 2 + plane];
+                    f.write(reinterpret_cast<const char*>(row.data()), static_cast<std::streamsize>(row.size() * sizeof(float)));
+                }
             }
         }
     } catch (const std::exception& e) {

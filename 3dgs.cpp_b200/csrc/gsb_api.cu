@@ -367,7 +367,7 @@ static int enqueue_front(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t rb, uin
 
 // k_blend over tile rows [b0, b1) of the frame; `band_out` is the first pixel row of the frame's band [fp.rb, fp.re).
 int enqueue_blend(gsb_ctx* ctx, const FramePlan& fp, uint32_t b0, uint32_t b1, void* band_out, size_t pitch, int fmt,
-                  cudaStream_t stream, void* const* peer_frames, int num_peer_frames) {
+                  cudaStream_t stream, void* const* peer_frames, int num_peer_frames, void* band_aux, size_t aux_pitch) {
     BlendParams bp{};
     bp.recs = ctx->recs;
     bp.vals = ctx->vals[fp.fin];
@@ -393,6 +393,10 @@ int enqueue_blend(gsb_ctx* ctx, const FramePlan& fp, uint32_t b0, uint32_t b1, v
     bp.stats = ctx->debug ? 2 : (ctx->timers ? 1 : 0);  // 2 also counts blend_pixel_hits (a few % of the kernel)
     bp.one = 1.0f;
     bp.ctl = ctx->ctl;
+    if (band_aux) {  // gsb_render_aux: the (opacity, depth) plane, same band layout as `band_out`
+        bp.aux = reinterpret_cast<float2*>(static_cast<unsigned char*>(band_aux) + (size_t)(b0 - fp.rb) * GSB_TILE * aux_pitch);
+        bp.aux_pitch = aux_pitch;
+    }
     CK(launch_blend(bp, stream));
     return GSB_OK;
 }
@@ -416,13 +420,13 @@ int enqueue_tail(gsb_ctx* ctx, const FramePlan& fp, cudaStream_t stream) {
     return GSB_OK;
 }
 
-// Enqueue one whole frame on `stream`; out_dev is device memory.
+// Enqueue one whole frame on `stream`; out_dev (and aux_dev, if not null) is device memory.
 static int enqueue_frame(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t rb, uint32_t re, void* out_dev, size_t pitch, int fmt,
-                  cudaStream_t stream) {
+                  cudaStream_t stream, void* aux_dev = nullptr, size_t aux_pitch = 0) {
     FramePlan fp{};
     int rc = enqueue_front(ctx, ubo, rb, re, stream, &fp);
     if (rc != GSB_OK) return rc;
-    rc = enqueue_blend(ctx, fp, rb, re, out_dev, pitch, fmt, stream);
+    rc = enqueue_blend(ctx, fp, rb, re, out_dev, pitch, fmt, stream, nullptr, 0, aux_dev, aux_pitch);
     if (rc != GSB_OK) return rc;
     return enqueue_tail(ctx, fp, stream);
 }
@@ -537,6 +541,7 @@ void gsb_destroy(gsb_ctx* ctx) {
     free_arena(ctx);
     dev_free(ctx->ranges);
     if (ctx->fb) cudaFree(ctx->fb);
+    if (ctx->aux_fb) cudaFree(ctx->aux_fb);
     dev_free(ctx->dbg_tiles);
     dev_free(ctx->dbg_aabb);
     dev_free(ctx->dbg_keys_unsorted);
@@ -751,47 +756,64 @@ int gsb_render_async(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t rb, uint32_
     return enqueue_frame(ctx, ubo, rb, re, out_device, pitch, fmt, s);
 }
 
-int gsb_render(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t rb, uint32_t re, void* out, size_t pitch, gsb_memory out_mem,
-               gsb_format fmt, void* stream) {
-    int rc = check_render_args(ctx, ubo, rb, re, out, pitch, fmt);
-    if (rc != GSB_OK) return rc;
+// Where the blend stores a HOST buffer of `need` bytes: a page-locked buffer (gsb_host_alloc / cudaHostAlloc / cudaHostRegister)
+// is written in place through its device alias; pageable memory goes through the device staging buffer (*buf, *bytes), grown
+// on demand, and one cudaMemcpy2D after the frame.
+static int host_target(gsb_ctx* ctx, void* host, size_t need, void** buf, size_t* bytes, void** dev, bool* staged) {
+    cudaPointerAttributes pa{};
+    const bool pinned = ctx->host_direct && cudaPointerGetAttributes(&pa, host) == cudaSuccess && pa.type == cudaMemoryTypeHost &&
+                        pa.devicePointer != nullptr;
+    cudaGetLastError();
+    *staged = !pinned;
+    if (pinned) {
+        *dev = pa.devicePointer;
+        return GSB_OK;
+    }
+    if (need > *bytes) {
+        if (*buf) cudaFree(*buf);
+        *buf = nullptr;
+        *bytes = 0;
+        CK(cudaMalloc(buf, need));
+        *bytes = need;
+    }
+    *dev = *buf;
+    return GSB_OK;
+}
+
+// gsb_render and gsb_render_aux: one synchronous frame, regrown and re-rendered on arena overflow.  aux == null: colour only.
+static int render_sync(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t rb, uint32_t re, void* out, size_t pitch, gsb_memory out_mem,
+                       gsb_format fmt, void* stream, void* aux, size_t aux_pitch) {
     CK(cudaSetDevice(ctx->device));
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
     const uint32_t H = ubo->height;
     const uint32_t rows = std::min(H, re * GSB_TILE) - rb * GSB_TILE;
     const size_t tight = (size_t)ubo->width * bytes_per_pixel(fmt);
+    const size_t aux_tight = (size_t)ubo->width * sizeof(float2);
+    int rc;
 
     // Host output.  If `out` is page-locked (gsb_host_alloc / cudaHostAlloc / cudaHostRegister) the blend stores the frame
     // straight into it over PCIe: k_blend2 writes whole 64-B tile rows, the stores are posted and the kernel is issue-bound,
     // so the 17.9 MB of a 3200x1400 BGRA8 frame leave the GPU while the blend is still running and no copy is left at the
     // end (the reference likewise stores into a host-visible swapchain image, render.comp:98).  Pageable memory goes
-    // through a device staging frame and one cudaMemcpy2D.
+    // through a device staging frame and one cudaMemcpy2D.  The aux plane is decided on its own: out and aux may differ.
     void* dev_out = out;
     size_t dev_pitch = pitch;
     bool staged = false;
+    void* dev_aux = aux;
+    size_t dev_aux_pitch = aux_pitch;
+    bool aux_staged = false;
     if (out_mem == GSB_MEM_HOST) {
-        cudaPointerAttributes pa{};
-        const bool pinned = ctx->host_direct && cudaPointerGetAttributes(&pa, out) == cudaSuccess &&
-                            pa.type == cudaMemoryTypeHost && pa.devicePointer != nullptr;
-        cudaGetLastError();
-        if (pinned) {
-            dev_out = pa.devicePointer;
-        } else {
-            const size_t need = tight * rows;
-            if (need > ctx->fb_bytes) {
-                if (ctx->fb) cudaFree(ctx->fb);
-                ctx->fb = nullptr;
-                ctx->fb_bytes = 0;
-                CK(cudaMalloc(&ctx->fb, need));
-                ctx->fb_bytes = need;
-            }
-            dev_out = ctx->fb;
-            dev_pitch = tight;
-            staged = true;
+        rc = host_target(ctx, out, tight * rows, &ctx->fb, &ctx->fb_bytes, &dev_out, &staged);
+        if (rc != GSB_OK) return rc;
+        if (staged) dev_pitch = tight;
+        if (aux) {
+            rc = host_target(ctx, aux, aux_tight * rows, &ctx->aux_fb, &ctx->aux_fb_bytes, &dev_aux, &aux_staged);
+            if (rc != GSB_OK) return rc;
+            if (aux_staged) dev_aux_pitch = aux_tight;
         }
     }
     for (int attempt = 0;; attempt++) {
-        rc = enqueue_frame(ctx, ubo, rb, re, dev_out, dev_pitch, fmt, s);
+        rc = enqueue_frame(ctx, ubo, rb, re, dev_out, dev_pitch, fmt, s, dev_aux, dev_aux_pitch);
         if (rc != GSB_OK) return rc;
         rc = wait_frame(ctx);
         if (rc != GSB_OK) return rc;
@@ -804,11 +826,30 @@ int gsb_render(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t rb, uint32_t re, 
         CK(cudaMemsetAsync(&ctx->ctl->overflow_sticky, 0, sizeof(uint32_t), s));  // this overflow is being handled right here
         ctx->regrow_count++;
     }
-    if (staged) {
-        CK(cudaMemcpy2DAsync(out, pitch, dev_out, dev_pitch, tight, rows, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
+    if (staged) CK(cudaMemcpy2DAsync(out, pitch, dev_out, dev_pitch, tight, rows, cudaMemcpyDeviceToHost, s));
+    if (aux_staged) CK(cudaMemcpy2DAsync(aux, aux_pitch, dev_aux, dev_aux_pitch, aux_tight, rows, cudaMemcpyDeviceToHost, s));
+    if (staged || aux_staged) CK(cudaStreamSynchronize(s));
     return GSB_OK;
+}
+
+int gsb_render(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t rb, uint32_t re, void* out, size_t pitch, gsb_memory out_mem,
+               gsb_format fmt, void* stream) {
+    int rc = check_render_args(ctx, ubo, rb, re, out, pitch, fmt);
+    if (rc != GSB_OK) return rc;
+    return render_sync(ctx, ubo, rb, re, out, pitch, out_mem, fmt, stream, nullptr, 0);
+}
+
+int gsb_render_aux(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t rb, uint32_t re, void* out, size_t pitch, float* aux,
+                   size_t aux_pitch, gsb_memory out_mem, gsb_format fmt, void* stream) {
+    if (!ctx) return GSB_ERR_INVALID;
+    if (!aux) return fail(ctx, GSB_ERR_INVALID, "null aux buffer");
+    if (ctx->shard) return fail(ctx, GSB_ERR_INVALID, "gsb_render_aux: aux planes are not available on a sharded context");
+    int rc = check_render_args(ctx, ubo, rb, re, out, pitch, fmt);
+    if (rc != GSB_OK) return rc;
+    const size_t aux_tight = (size_t)ubo->width * sizeof(float2);
+    if (aux_pitch == 0) aux_pitch = aux_tight;
+    if (aux_pitch < aux_tight || aux_pitch % sizeof(float2) != 0) return fail(ctx, GSB_ERR_INVALID, "bad aux row pitch");
+    return render_sync(ctx, ubo, rb, re, out, pitch, out_mem, fmt, stream, aux, aux_pitch);
 }
 
 int gsb_get_stats(gsb_ctx* ctx, gsb_stats* out) {

@@ -374,6 +374,16 @@ struct __align__(16) StagedRec2 {  // 80 B: five 16-B slots = five LDS.128 per v
     float4 q3;  // r r g g
     float4 q4;  // b b power_cut bits(index in batch)
 };
+struct __align__(16) StagedRec2Aux {  // 96 B (gsb_render_aux): StagedRec2 + a sixth slot
+    float4 q0, q1, q2, q3, q4;
+    float4 q5;  // depth depth - -     (view-space z = VertexAttribute.depth, pre-broadcast like the others)
+};
+template <bool AUX> struct StagedRec2Of { typedef StagedRec2 type; };
+template <> struct StagedRec2Of<true> { typedef StagedRec2Aux type; };
+
+#ifndef GSB_BLEND2_AUX_MIN_BLOCKS
+#define GSB_BLEND2_AUX_MIN_BLOCKS 7  // AUX: 72-register cap (the colour-only kernels sit at the 64-register cap of 8 CTAs/SM)
+#endif
 
 __device__ __forceinline__ uint32_t block_mask2(float ux, float uy, float A, float B, float C, float cut, float tile_x0, float tile_y0) {
     if (!(A > 0.0f) || !(C > 0.0f)) return 0xfu;  // not positive definite / NaN: never cull
@@ -413,9 +423,14 @@ __device__ __forceinline__ void exp_shared2(u64 x, u64 one2, float& e0, float& e
 // entries at a time (keys + payloads only, coalesced), keeps the entries whose mask has this tile's bit -- in list order, so
 // the tile's own (depth, index) order is preserved -- and gathers records only for those, until the batch holds up to
 // B2_BATCH of them.  The walk is unchanged.
-template <int MODE, bool STATS, bool COARSE>
-__global__ void __launch_bounds__(B2_THREADS, GSB_BLEND2_MIN_BLOCKS) k_blend2(const __grid_constant__ BlendParams P) {
-    __shared__ StagedRec2 s_rec[B2_BATCH];
+// AUX (gsb_render_aux): the walk also accumulates D += (depth * alpha) * T next to the colour and keeps the transmittance after
+// the last accumulated Gaussian (T itself is overwritten with 0 at the break); every pixel then stores (1 - T_end, D).  All
+// of it sits behind `if constexpr (AUX)`: the colour-only instantiations are unchanged.
+template <int MODE, bool STATS, bool COARSE, bool AUX>
+__global__ void __launch_bounds__(B2_THREADS, AUX ? GSB_BLEND2_AUX_MIN_BLOCKS : GSB_BLEND2_MIN_BLOCKS)
+    k_blend2(const __grid_constant__ BlendParams P) {
+    typedef typename StagedRec2Of<AUX>::type Rec;
+    __shared__ Rec s_rec[B2_BATCH];
     __shared__ uint8_t s_mask[B2_BATCH];
     __shared__ uint32_t s_wc[B2_WARPS];
 #if GSB_BLEND_TMA
@@ -432,7 +447,7 @@ __global__ void __launch_bounds__(B2_THREADS, GSB_BLEND2_MIN_BLOCKS) k_blend2(co
     uint32_t* const s_cid = reinterpret_cast<uint32_t*>(&s_list[0][0]);
     uint32_t* const s_eidx = s_cid + B2_BATCH;
     __shared__ uint32_t s_used, s_walked, s_hits;
-    static_assert(sizeof(StagedRec2) * B2_BATCH < 65536, "u16 list entries hold shared-window addresses");
+    static_assert(sizeof(Rec) * B2_BATCH < 65536, "u16 list entries hold shared-window addresses");
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t tx = blockIdx.x % P.tiles_x;
@@ -459,6 +474,8 @@ __global__ void __launch_bounds__(B2_THREADS, GSB_BLEND2_MIN_BLOCKS) k_blend2(co
     // transmittance (0 = finished or outside the image) and colour a/b/c of pixel 0/1
     float T0 = in0 ? 1.0f : 0.0f, T1 = in1 ? 1.0f : 0.0f, ca0 = 0.f, ca1 = 0.f, cb0 = 0.f, cb1 = 0.f, cc0 = 0.f, cc1 = 0.f;
 #define B2_DONE (T0 == 0.0f && T1 == 0.0f)
+    // AUX: expected depth and the transmittance after the last accumulated Gaussian (T0 / T1 become 0 at the break)
+    float d0 = 0.f, d1 = 0.f, tl0 = 1.0f, tl1 = 1.0f;
     uint32_t used = 0, walked = 0, hits = 0, staged = 0;
     const uint32_t rec_sh = (uint32_t)__cvta_generic_to_shared(&s_rec[0]);
     const uint32_t list_sh = (uint32_t)__cvta_generic_to_shared(&s_list[warp][0]);
@@ -579,6 +596,7 @@ __global__ void __launch_bounds__(B2_THREADS, GSB_BLEND2_MIN_BLOCKS) k_blend2(co
                     s_rec[li].q3 = make_float4(col.x, col.x, col.y, col.y);
                     // q4.w: position in the list relative to the batch's base offset (the consumed-entries statistic)
                     s_rec[li].q4 = make_float4(col.z, col.z, cut, __uint_as_float(COARSE ? s_eidx[li] : li));
+                    if constexpr (AUX) s_rec[li].q5 = make_float4(col.w, col.w, 0.f, 0.f);  // q2.w of the record: view-space depth
                 }
                 s_mask[li] = (uint8_t)m;
             }
@@ -589,7 +607,7 @@ __global__ void __launch_bounds__(B2_THREADS, GSB_BLEND2_MIN_BLOCKS) k_blend2(co
             for (uint32_t c = 0; c < cnt; c += 32) {  // one ballot per 32 records
                 const bool mine = (c + lane < cnt) && ((s_mask[c + lane] >> warp) & 1u);
                 const unsigned bits = __ballot_sync(FULL, mine);
-                if (mine) s_list[warp][n + __popc(bits & ((1u << lane) - 1u))] = (uint16_t)(rec_sh + (c + lane) * sizeof(StagedRec2));
+                if (mine) s_list[warp][n + __popc(bits & ((1u << lane) - 1u))] = (uint16_t)(rec_sh + (c + lane) * sizeof(Rec));
                 n += __popc(bits);
             }
             __syncwarp();
@@ -644,6 +662,24 @@ __global__ void __launch_bounds__(B2_THREADS, GSB_BLEND2_MIN_BLOCKS) k_blend2(co
                         const uint32_t u = base_off + __float_as_uint(idxf) + 1u;
                         used = ((in0k && !ok0 && T0 != 0.0f) || (in1k && !ok1 && T1 != 0.0f)) ? max(used, u) : used;
                         if (P.stats > 1) hits += (in0k && T0 != 0.0f ? 1u : 0u) + (in1k && T1 != 0.0f ? 1u : 0u);  // debug frames only
+                    }
+                    if constexpr (AUX) {
+                        u64 z2, zpad;
+                        lds_2x64(addr + 80u, z2, zpad);
+                        float wd0, wd1;
+                        if (MODE == GSB_MODE_EXACT) {
+                            upk2(mul2(mul2(z2, alpha2), T2), wd0, wd1);  // (depth * alpha) * T, :87's shape
+                            if (ok0) d0 = __fadd_rn(d0, wd0);
+                            if (ok1) d1 = __fadd_rn(d1, wd1);
+                        } else {
+                            float z, z_;
+                            upk2(z2, z, z_);
+                            upk2(mul2(alpha2, T2), wd0, wd1);
+                            if (ok0) d0 = fmaf(z, wd0, d0);
+                            if (ok1) d1 = fmaf(z, wd1, d1);
+                        }
+                        tl0 = ok0 ? tt0 : tl0;  // :88 without the break's 0
+                        tl1 = ok1 ? tt1 : tl1;
                     }
 #if GSB_BLEND2_PRED
                     // predicated scalar accumulates (FMA pipe) instead of packed adds + selects (the half-rate ALU pipe is
@@ -754,6 +790,11 @@ __global__ void __launch_bounds__(B2_THREADS, GSB_BLEND2_MIN_BLOCKS) k_blend2(co
             }
         }
     }
+    if constexpr (AUX) {  // one 8-B store per pixel: the 8 lanes of a pixel row cover 64 contiguous bytes
+        unsigned char* abase = reinterpret_cast<unsigned char*>(P.aux);
+        if (in0) reinterpret_cast<float2*>(abase + (size_t)row0 * P.aux_pitch)[px] = make_float2(__fsub_rn(1.0f, tl0), d0);
+        if (in1) reinterpret_cast<float2*>(abase + (size_t)(row0 + 4) * P.aux_pitch)[px] = make_float2(__fsub_rn(1.0f, tl1), d1);
+    }
     if (STATS) {
         __syncthreads();
         if (tid == 0) {
@@ -765,29 +806,38 @@ __global__ void __launch_bounds__(B2_THREADS, GSB_BLEND2_MIN_BLOCKS) k_blend2(co
     }
 }
 
+template <bool AUX>
+void launch_blend2(const BlendParams& p, uint32_t blocks, cudaStream_t s) {
+    if (p.coarse_shift) {
+        if (p.stats) {
+            if (p.mode == GSB_MODE_EXACT) k_blend2<GSB_MODE_EXACT, true, true, AUX><<<blocks, B2_THREADS, 0, s>>>(p);
+            else k_blend2<GSB_MODE_FAST, true, true, AUX><<<blocks, B2_THREADS, 0, s>>>(p);
+        } else {
+            if (p.mode == GSB_MODE_EXACT) k_blend2<GSB_MODE_EXACT, false, true, AUX><<<blocks, B2_THREADS, 0, s>>>(p);
+            else k_blend2<GSB_MODE_FAST, false, true, AUX><<<blocks, B2_THREADS, 0, s>>>(p);
+        }
+    } else if (p.stats) {
+        if (p.mode == GSB_MODE_EXACT) k_blend2<GSB_MODE_EXACT, true, false, AUX><<<blocks, B2_THREADS, 0, s>>>(p);
+        else k_blend2<GSB_MODE_FAST, true, false, AUX><<<blocks, B2_THREADS, 0, s>>>(p);
+    } else {
+        if (p.mode == GSB_MODE_EXACT) k_blend2<GSB_MODE_EXACT, false, false, AUX><<<blocks, B2_THREADS, 0, s>>>(p);
+        else k_blend2<GSB_MODE_FAST, false, false, AUX><<<blocks, B2_THREADS, 0, s>>>(p);
+    }
+}
+
 }  // namespace
 
 cudaError_t launch_blend(const BlendParams& p, cudaStream_t s) {
     const uint32_t rows = p.tile_row_end - p.tile_row_begin;
     const uint32_t blocks = rows * p.tiles_x;
     if (blocks == 0) return cudaSuccess;
-    if (p.variant == 1 && p.num_peers == 0 && p.coarse_shift == 0) {  // round-1 kernel (one pixel per thread), kept for A/B: GSB_BLEND_VARIANT=1
+    if (p.aux) {  // gsb_render_aux (single context only): k_blend2, the round-1 kernel has no aux planes
+        launch_blend2<true>(p, blocks, s);
+    } else if (p.variant == 1 && p.num_peers == 0 && p.coarse_shift == 0) {  // round-1 kernel (one pixel per thread), kept for A/B: GSB_BLEND_VARIANT=1
         if (p.mode == GSB_MODE_EXACT) k_blend<GSB_MODE_EXACT><<<blocks, BLEND_THREADS, 0, s>>>(p);
         else k_blend<GSB_MODE_FAST><<<blocks, BLEND_THREADS, 0, s>>>(p);
-    } else if (p.coarse_shift) {
-        if (p.stats) {
-            if (p.mode == GSB_MODE_EXACT) k_blend2<GSB_MODE_EXACT, true, true><<<blocks, B2_THREADS, 0, s>>>(p);
-            else k_blend2<GSB_MODE_FAST, true, true><<<blocks, B2_THREADS, 0, s>>>(p);
-        } else {
-            if (p.mode == GSB_MODE_EXACT) k_blend2<GSB_MODE_EXACT, false, true><<<blocks, B2_THREADS, 0, s>>>(p);
-            else k_blend2<GSB_MODE_FAST, false, true><<<blocks, B2_THREADS, 0, s>>>(p);
-        }
-    } else if (p.stats) {
-        if (p.mode == GSB_MODE_EXACT) k_blend2<GSB_MODE_EXACT, true, false><<<blocks, B2_THREADS, 0, s>>>(p);
-        else k_blend2<GSB_MODE_FAST, true, false><<<blocks, B2_THREADS, 0, s>>>(p);
     } else {
-        if (p.mode == GSB_MODE_EXACT) k_blend2<GSB_MODE_EXACT, false, false><<<blocks, B2_THREADS, 0, s>>>(p);
-        else k_blend2<GSB_MODE_FAST, false, false><<<blocks, B2_THREADS, 0, s>>>(p);
+        launch_blend2<false>(p, blocks, s);
     }
     return cudaGetLastError();
 }

@@ -61,6 +61,8 @@ struct gsb_ctx {
     uint32_t ranges_tiles = 0;
     void* fb = nullptr;
     size_t fb_bytes = 0;
+    void* aux_fb = nullptr;  // gsb_render_aux: device staging of a pageable host aux plane
+    size_t aux_fb_bytes = 0;
 
     int mode = GSB_MODE_EXACT;
     bool debug = false;
@@ -142,7 +144,8 @@ int plan_frame(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t rb, uint32_t re, 
 int enqueue_middle(gsb_ctx* ctx, const FramePlan& fp, cudaStream_t stream, bool events);
 int launch_middle_graph(gsb_ctx* ctx, const FramePlan& fp, cudaStream_t stream);
 int enqueue_blend(gsb_ctx* ctx, const FramePlan& fp, uint32_t b0, uint32_t b1, void* band_out, size_t pitch, int fmt,
-                  cudaStream_t stream, void* const* peer_frames = nullptr, int num_peer_frames = 0);
+                  cudaStream_t stream, void* const* peer_frames = nullptr, int num_peer_frames = 0, void* band_aux = nullptr,
+                  size_t aux_pitch = 0);
 int enqueue_tail(gsb_ctx* ctx, const FramePlan& fp, cudaStream_t stream);
 int check_render_args(gsb_ctx* ctx, const gsb_uniforms* ubo, uint32_t& rb, uint32_t& re, const void* out, size_t& pitch, int fmt);
 

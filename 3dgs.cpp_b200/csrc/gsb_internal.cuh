@@ -155,6 +155,10 @@ struct BlendParams {
     int stats;              // 1: count blend_consumed / blend_walked (~4 instructions per record); 2: blend_hits as well
     float one;              // 1.0f, passed as data so that ptxas cannot fold it (gsb_blend.cu, add2_of_product)
     Control* ctl;
+    // gsb_render_aux: per-pixel (opacity, expected depth) plane, laid out like `out` (pixel row `out_first_row` at aux + 0,
+    // rows aux_pitch bytes apart); null = colour only.  Single-context frames only (num_peers == 0).
+    float2* aux;
+    size_t aux_pitch;
 };
 cudaError_t launch_blend(const BlendParams& p, cudaStream_t s);
 

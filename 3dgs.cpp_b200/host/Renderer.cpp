@@ -114,6 +114,20 @@ const void* Renderer::render(uint32_t width, uint32_t height, gsb_format format)
     return hostFrame.data();
 }
 
+const float* Renderer::renderAux(uint32_t width, uint32_t height, gsb_format format) {
+    if (!ctx) throw std::runtime_error("Renderer::renderAux before initialize()");
+    const UniformBuffer ubo = makeUniforms(camera, width, height);
+    const size_t bpp = format == GSB_FORMAT_RGBA32F ? 16 : 4;
+    hostFrame.resize(static_cast<size_t>(width) * height * bpp);
+    hostAux.resize(static_cast<size_t>(width) * height * 2 * sizeof(float));
+    gsb_uniforms u;
+    std::memcpy(&u, &ubo, sizeof u);
+    check(gsb_render_aux(ctx, &u, 0, UINT32_MAX, hostFrame.data(), 0, reinterpret_cast<float*>(hostAux.data()), 0, GSB_MEM_HOST,
+                         format, nullptr),
+          "gsb_render_aux");
+    return reinterpret_cast<const float*>(hostAux.data());
+}
+
 void Renderer::draw() { render(configuration.width, configuration.height, configuration.format); }
 
 void Renderer::run(uint32_t frames) {

@@ -72,6 +72,9 @@ public:
     // Render at an explicit size; returns tightly packed RGBA32F / RGBA8 / BGRA8 pixels owned by the renderer.
     const void* render(uint32_t width, uint32_t height, gsb_format format);
     const void* render(uint32_t width, uint32_t height) { return render(width, height, GSB_FORMAT_RGBA32F); }
+    // render() plus the frame's per-pixel (opacity, expected depth) planes (gsb_render_aux): the pixels go to frame() as with
+    // render(); returns width * height float2, page-locked and owned by the renderer (auxFrame()).
+    const float* renderAux(uint32_t width, uint32_t height, gsb_format format);
     // The last frame.  The buffer is page-locked (gsb_host_alloc): gsb_render's blend stores the pixels straight into it over
     // PCIe while it runs -- the analogue of the reference's host-visible swapchain image (render.comp:98) -- instead of a
     // device frame + a pageable cudaMemcpy (measured 16 ms per 3200x1400 BGRA8 frame through a std::vector).
@@ -89,6 +92,7 @@ public:
         HostFrame& operator=(const HostFrame&) = delete;
     };
     const HostFrame& frame() const { return hostFrame; }
+    const HostFrame& auxFrame() const { return hostAux; }  // planes of the last renderAux()
 
     // Renderer::updateUniforms (Renderer.cpp:719-754), exposed so tests can pin it.
     static UniformBuffer makeUniforms(const Camera& camera, uint32_t width, uint32_t height);
@@ -110,6 +114,7 @@ private:
     gsb_ctx* ctx = nullptr;
     std::shared_ptr<GSScene> scene;
     HostFrame hostFrame;
+    HostFrame hostAux;
     std::atomic<bool> running{true};
     void check(int rc, const char* what);
 };

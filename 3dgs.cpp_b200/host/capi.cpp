@@ -112,6 +112,16 @@ int gsh_render(gsh_renderer* r, uint32_t width, uint32_t height, int format, voi
         }
     });
 }
+int gsh_render_aux(gsh_renderer* r, uint32_t width, uint32_t height, int format, void* out, size_t out_bytes, float* aux,
+                   size_t aux_bytes) {
+    return guard([&] {
+        const float* planes = r->r->renderAux(width, height, static_cast<gsb_format>(format));
+        const size_t need = r->r->frame().size(), need_aux = r->r->auxFrame().size();
+        if ((out && out_bytes < need) || (aux && aux_bytes < need_aux)) throw std::runtime_error("gsh_render_aux: output buffer too small");
+        if (out) std::memcpy(out, r->r->frame().data(), need);
+        if (aux) std::memcpy(aux, planes, need_aux);
+    });
+}
 const void* gsh_frame(gsh_renderer* r, size_t* bytes) {
     if (bytes) *bytes = r->r->frame().size();
     return r->r->frame().data();

@@ -37,6 +37,10 @@ int gsh_set_camera(gsh_renderer *r, const float pos[3], const float quat_wxyz[4]
 int gsh_get_camera(gsh_renderer *r, float pos[3], float quat_wxyz[4], float *fov_deg);
 int gsh_key_input(gsh_renderer *r, const int keys[6]); /* W A S D space shift for one handleInput() */
 int gsh_render(gsh_renderer *r, uint32_t width, uint32_t height, int format, void *out, size_t out_bytes);
+/* Renderer::renderAux: gsh_render + the width*height float2 (opacity, expected depth) planes of gsb_render_aux into aux
+ * (aux_bytes >= 8 * width * height; either buffer may be NULL to leave it in the renderer) */
+int gsh_render_aux(gsh_renderer *r, uint32_t width, uint32_t height, int format, void *out, size_t out_bytes, float *aux,
+                   size_t aux_bytes);
 const void *gsh_frame(gsh_renderer *r, size_t *bytes); /* pixels of the last draw()/render() */
 int gsh_stats(gsh_renderer *r, gsb_stats *out);
 uint64_t gsh_num_vertices(gsh_renderer *r);

@@ -38,7 +38,7 @@ ALL_ROWS = 0xFFFFFFFF
 EXPORTED_SYMBOLS = [  # every symbol include/gs_b200.h declares
     "gsb_abi_version", "gsb_device_count", "gsb_create", "gsb_destroy", "gsb_last_error",
     "gsb_scene_upload", "gsb_scene_size", "gsb_set_mode", "gsb_set_debug", "gsb_set_timers", "gsb_set_tile_cull", "gsb_set_sh_storage",
-    "gsb_reserve_instances", "gsb_render", "gsb_render_async", "gsb_get_stats", "gsb_debug_size",
+    "gsb_reserve_instances", "gsb_render", "gsb_render_aux", "gsb_render_async", "gsb_get_stats", "gsb_debug_size",
     "gsb_debug_download", "gsb_sort_pairs", "gsb_sort_pairs32", "gsb_set_graph", "gsb_host_alloc", "gsb_host_free",
     # frame sharding over several GPUs
     "gsb_group_create", "gsb_group_destroy", "gsb_group_size", "gsb_group_context", "gsb_group_last_error",
@@ -48,7 +48,7 @@ EXPORTED_SYMBOLS = [  # every symbol include/gs_b200.h declares
 ]
 HOST_EXPORTED_SYMBOLS = [  # host/gs_b200_host.h
     "gsh_last_error", "gsh_initialize", "gsh_draw", "gsh_pan_translation", "gsh_movement", "gsh_cleanup",
-    "gsh_set_camera", "gsh_get_camera", "gsh_key_input", "gsh_render", "gsh_frame", "gsh_stats",
+    "gsh_set_camera", "gsh_get_camera", "gsh_key_input", "gsh_render", "gsh_render_aux", "gsh_frame", "gsh_stats",
     "gsh_num_vertices", "gsh_context", "gsh_uniforms_from_camera", "gsh_camera_translate",
     "gsh_activate_records", "gsh_load_ply", "gsh_free", "gsh_write_ply", "gsh_synth_default_params",
     "gsh_synth_records",
@@ -111,6 +111,8 @@ lib.gsb_host_free.argtypes = [_vp]
 lib.gsb_host_free.restype = None
 lib.gsb_reserve_instances.argtypes = [_vp, C.c_uint64]
 lib.gsb_render.argtypes = [_vp, C.POINTER(Uniforms), C.c_uint32, C.c_uint32, _vp, C.c_size_t, C.c_int, C.c_int, _vp]
+lib.gsb_render_aux.argtypes = [_vp, C.POINTER(Uniforms), C.c_uint32, C.c_uint32, _vp, C.c_size_t, _vp, C.c_size_t, C.c_int,
+                                C.c_int, _vp]
 lib.gsb_render_async.argtypes = [_vp, C.POINTER(Uniforms), C.c_uint32, C.c_uint32, _vp, C.c_size_t, C.c_int, _vp]
 lib.gsb_get_stats.argtypes = [_vp, C.POINTER(Stats)]
 lib.gsb_debug_size.argtypes = [_vp, C.c_int]
@@ -155,6 +157,7 @@ host.gsh_cleanup.restype = None
 host.gsh_set_camera.argtypes = [_vp, _vp, _vp, C.c_float, C.c_float, C.c_float]
 host.gsh_get_camera.argtypes = [_vp, _vp, _vp, C.POINTER(C.c_float)]
 host.gsh_render.argtypes = [_vp, C.c_uint32, C.c_uint32, C.c_int, _vp, C.c_size_t]
+host.gsh_render_aux.argtypes = [_vp, C.c_uint32, C.c_uint32, C.c_int, _vp, C.c_size_t, _vp, C.c_size_t]
 host.gsh_frame.argtypes = [_vp, C.POINTER(C.c_size_t)]
 host.gsh_frame.restype = _vp
 host.gsh_stats.argtypes = [_vp, C.POINTER(Stats)]
@@ -354,6 +357,22 @@ class Context:
         else:
             self._ck(lib.gsb_render_async(self.h, C.byref(u), rb, re, out_ptr, 0, fmt, stream_ptr(stream)))
 
+    def render_aux(self, u: Uniforms, fmt=FORMAT_RGBA32F, rows=None):
+        """gsb_render_aux to HOST numpy arrays: (img, aux) with aux of shape (rows, W, 2) float32 = (opacity, expected depth)
+        per pixel; img is exactly what render() returns."""
+        rb, re, nrows = self.band_rows(u, rows)
+        out = np.empty((nrows, u.width, 4), np.float32 if fmt == FORMAT_RGBA32F else np.uint8)
+        aux = np.empty((nrows, u.width, 2), np.float32)
+        self._ck(lib.gsb_render_aux(self.h, C.byref(u), rb, re, out.ctypes.data, 0, aux.ctypes.data, 0, MEM_HOST, fmt, None))
+        return out, aux
+
+    def render_aux_into(self, u: Uniforms, out_ptr: int, aux_ptr: int, fmt=FORMAT_RGBA32F, rows=None, stream=None,
+                        aux_row_pitch=0):
+        """gsb_render_aux into DEVICE memory (e.g. tensor.data_ptr()); aux_row_pitch in bytes, 0 = tight."""
+        rb, re, _ = self.band_rows(u, rows)
+        self._ck(lib.gsb_render_aux(self.h, C.byref(u), rb, re, out_ptr, 0, aux_ptr, aux_row_pitch, MEM_DEVICE, fmt,
+                                    stream_ptr(stream)))
+
     def stats(self) -> Stats:
         s = Stats()
         self._ck(lib.gsb_get_stats(self.h, C.byref(s)))
@@ -532,6 +551,14 @@ class HostRenderer:
     def render(self, width, height, fmt=FORMAT_RGBA32F) -> np.ndarray:
         self._ck(host.gsh_render(self.h, width, height, fmt, None, 0))
         return self._frame(width, height, fmt)
+
+    def render_aux(self, width, height, fmt=FORMAT_RGBA32F):
+        """Renderer::renderAux: (img, aux) with aux of shape (height, width, 2) float32 = (opacity, expected depth)."""
+        dt = np.float32 if fmt == FORMAT_RGBA32F else np.uint8
+        img = np.empty((height, width, 4), dt)
+        aux = np.empty((height, width, 2), np.float32)
+        self._ck(host.gsh_render_aux(self.h, width, height, fmt, img.ctypes.data, img.nbytes, aux.ctypes.data, aux.nbytes))
+        return img, aux
 
     def _frame(self, w, h, fmt):
         n = C.c_size_t()

@@ -197,6 +197,23 @@ int gsb_reserve_instances(gsb_ctx *ctx, uint64_t capacity);
 int gsb_render(gsb_ctx *ctx, const gsb_uniforms *ubo, uint32_t tile_row_begin, uint32_t tile_row_end,
                void *out, size_t row_pitch_bytes, gsb_memory out_mem, gsb_format fmt, void *stream);
 
+/* gsb_render plus two per-pixel planes of the same frame, for compositing and depth testing (no reference counterpart:
+ * render.comp:98 stores vec4(c, 1) and drops the transmittance).  `out` receives exactly what gsb_render writes.  `aux`
+ * receives one float2 (x = opacity, y = expected depth) per pixel for the same pixel rows, `aux_row_pitch_bytes` apart
+ * (0 = tight, 8 * width; otherwise >= 8 * width and a multiple of 8).  out_mem applies to both buffers; each one may be
+ * page-locked or pageable on its own.  Walking the tile's list as render.comp:61-89 does, a Gaussian i is *accumulated*
+ * when it reaches :87 (passes :68-70 and :78-80 and does not trigger the break at :83-85); T_i is T just before it:
+ *   opacity = 1 - T_end (one fp32 subtraction), T_end = T after the last accumulated Gaussian; in [0, 0.9999], 0 if none;
+ *   depth   = D, D = D + (depth_i * alpha_i) * T_i in list order (the shape of :87), depth_i = VertexAttribute.depth (the
+ *             view-space z of GSB_BUF_ATTR).  D is NOT normalised: the mean depth of the covered part is depth / opacity.
+ * The colour is premultiplied, so the frame over a background B is c + (1 - opacity) * B.  EXACT mode: both planes are
+ * bit-identical to the oracle with exp mode 1 and the colour to gsb_render's; FAST mode accumulates D = fma(depth, alpha*T, D).
+ * Errors: GSB_ERR_INVALID for a null aux, a bad aux pitch, or a context of a sharded frame (gsb_create_sharded,
+ * gsb_group_context); everything else as gsb_render. */
+int gsb_render_aux(gsb_ctx *ctx, const gsb_uniforms *ubo, uint32_t tile_row_begin, uint32_t tile_row_end,
+                   void *out, size_t row_pitch_bytes, float *aux, size_t aux_row_pitch_bytes,
+                   gsb_memory out_mem, gsb_format fmt, void *stream);
+
 /* Enqueue-only variant for pipelined callers (bench e2e): never synchronises, never regrows;
  * overflow is reported by the next gsb_get_stats()/gsb_render().  out must be device memory. */
 int gsb_render_async(gsb_ctx *ctx, const gsb_uniforms *ubo, uint32_t tile_row_begin,
